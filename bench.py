@@ -7,6 +7,7 @@ softmax weighted mean + update.  value = Nsample*Hsample / t_step, whole job ove
 
   python bench.py [--gpus N --steps K --warmup W]        # under torchrun for N > 1
   python bench.py --impl reference ...                   # the CPU restatement (oracle) arm
+  python bench.py --dump-outputs DIR ...                 # also save what the last timed step computed, for comparing builds
 
 Timing: CUDA events recorded on the launching stream by the C launch sequence itself (before the step, after the
 rollout kernel, after the step), >= 3 warm-ups, L2 flushed (256 MiB memset, untimed) between steps, barrier +
@@ -35,6 +36,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 ENV_NAME, NSAMPLE, HSAMPLE, NDIFFUSE, TEMP = "humanoidrun", 8192, 50, 300, 0.1
 NU, NFRAMES = 17, 7
@@ -267,14 +269,20 @@ def run_gpu(args):
         return tot, kern, kw
 
     breakdown = {}
+    outputs = {}
 
-    def measure(n_total):
-        """(ms per step, rollout-kernel ms, e2e ms per step, parity_ok or None, engine) for n_total samples over `world` ranks"""
+    def measure(n_total, keep_outputs=False):
+        """(ms per step, rollout-kernel ms, e2e ms per step, parity_ok or None, engine) for n_total samples over `world` ranks;
+        keep_outputs: copy what the last timed step returned into `outputs` before later steps overwrite it"""
         e = make_engine(n_total)
         chain(e, args.warmup, False, False)
         barrier()
         tot, kern, kw = chain(e, args.steps, True, False)
         barrier()
+        if keep_outputs:
+            i = int(e.ctl[0].item()) + 1     # the last timed step read Ybars[i] and wrote Ybars[i - 1]
+            outputs.update(ybar_im1=e.Ybars[i - 1].view(HSAMPLE, NU).cpu().numpy(), rew_mean=e.rew_hist[i].cpu().numpy(),
+                           returns=e.rews_all.cpu().numpy())
         chain(e, 1, False, True)
         barrier()
         e2e, _, _ = chain(e, args.steps, True, True)
@@ -311,9 +319,14 @@ def run_gpu(args):
     if rank == 0:
         sampler.start()
     n_weak = NSAMPLE * world if args.scaling == "weak" else NSAMPLE
-    ms_step, kern_ms, e2e_ms, parity_ok, e = measure(n_weak)
+    ms_step, kern_ms, e2e_ms, parity_ok, e = measure(n_weak, keep_outputs=bool(args.dump_outputs))
     weak_breakdown = dict(breakdown)
     clocks = sampler.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        # float32; the chain is the fixed seed-0 one, so the same arguments give the same inputs on every run and every build
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in outputs.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     n_local = e.n_local
     del e
     strong = None
@@ -423,11 +436,14 @@ def main():
     ap.add_argument("--cpu-samples", type=int, default=4096)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-solve", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
     if 2 * args.steps + args.warmup + 2 >= NDIFFUSE:
         raise SystemExit("2*steps + warmup + 2 must be < Ndiffuse")
     if args.impl == "reference":
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs saves the outputs of the GPU arm; --impl reference times a sample of the rollouts only")
         run_reference(args)
     else:
         run_gpu(args)

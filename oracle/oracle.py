@@ -36,17 +36,30 @@ def build(force: bool = False) -> str:
     return so
 
 
+_HOST_DIR = None
+
+
+def _host_build_dir() -> str:
+    """Scratch directory of this process for the libraries compiled for THIS host at run time (-march=native).  They
+    never go into the source tree, which may be read-only where bench.py runs; the directory is removed at exit."""
+    global _HOST_DIR
+    if _HOST_DIR is None:
+        import atexit
+        import shutil
+        import tempfile
+        _HOST_DIR = tempfile.mkdtemp(prefix="mbd_oracle_")
+        atexit.register(shutil.rmtree, _HOST_DIR, True)
+    return _HOST_DIR
+
+
 def use_native() -> bool:
-    """Switches this process to oracle/libmbd_oracle_native.so: the same source built `-O3 -march=native` ON THIS HOST
+    """Switches this process to libmbd_oracle_native.so: the same source built `-O2 -march=native` ON THIS HOST
     (bench.py's timed CPU arm; -ffp-contract=off is kept, so the results are the same bits).  Returns False — and keeps
     the portable build — when the compile fails."""
     global _LIB
-    import fcntl
-    so = os.path.join(_HERE, "libmbd_oracle_native.so")
+    so = os.path.join(_host_build_dir(), "libmbd_oracle_native.so")
     try:
-        with open(os.path.join(_HERE, ".build.lock"), "w") as lock:
-            fcntl.flock(lock, fcntl.LOCK_EX)
-            subprocess.run(["make", "-C", _HERE, "-B", "native"], check=True, capture_output=True)
+        subprocess.run(["make", "-C", _HERE, "-B", "native", "NATIVE_OUT=" + so], check=True, capture_output=True)
         L = ctypes.CDLL(so)
         L.orc_num_threads.restype = ctypes.c_int
         _LIB = L
@@ -59,15 +72,14 @@ _SIMD = None
 
 
 def use_simd():
-    """Builds (on THIS host, -march=native) and loads oracle/libmbd_oracle_simd.so — the SIMD-across-samples CPU arm of
+    """Builds (on THIS host, -march=native) and loads libmbd_oracle_simd.so — the SIMD-across-samples CPU arm of
     bench.py (mbd_oracle_simd.cpp: the templated physics of csrc/xpbd_pk.cuh instantiated with a 16-lane host type; same
     bits as the scalar oracle).  Returns the library or None when it cannot be built."""
     global _SIMD
     if _SIMD is not None:
         return _SIMD or None
-    import fcntl
     root = os.path.join(_HERE, "..")
-    so = os.path.join(_HERE, "libmbd_oracle_simd.so")
+    so = os.path.join(_host_build_dir(), "libmbd_oracle_simd.so")
     flags = ["-O3", "-march=native", "-std=c++17", "-ffp-contract=off", "-fno-math-errno", "-fopenmp", "-shared", "-fPIC", "-fvisibility=hidden"]
     try:
         with open("/proc/cpuinfo") as f:
@@ -76,10 +88,8 @@ def use_simd():
     except OSError:
         pass
     try:
-        with open(os.path.join(_HERE, ".build.lock"), "w") as lock:
-            fcntl.flock(lock, fcntl.LOCK_EX)
-            subprocess.run(["g++"] + flags + ["-I" + os.path.join(root, "include"), "-I" + os.path.join(root, "mbd_b200", "csrc"),
-                                              os.path.join(_HERE, "mbd_oracle_simd.cpp"), "-o", so], check=True, capture_output=True)
+        subprocess.run(["g++"] + flags + ["-I" + os.path.join(root, "include"), "-I" + os.path.join(root, "mbd_b200", "csrc"),
+                                          os.path.join(_HERE, "mbd_oracle_simd.cpp"), "-o", so], check=True, capture_output=True)
         _SIMD = ctypes.CDLL(so)
     except Exception:  # noqa: BLE001
         _SIMD = False

@@ -30,6 +30,8 @@ typedef void* mbd_stream; /* cudaStream_t */
 int mbd_layout_info(int32_t* out, int n);
 /* sizeof / offsetof of the structs passed by pointer (mbd_step_params, mbd_step_ctl, mbd_step_plan), same cross-check */
 int mbd_abi_sizes(int32_t* out, int n);
+/* offsetof(mbd_step_plan, n_solves / n_diffuse / temps_dev): the batched-solve fields, same cross-check */
+int mbd_abi_batch_offsets(int32_t* out, int n);
 const char* mbd_last_error(void);
 int mbd_device_count(void);
 /* rollout kernel mapping: 0 = auto (by shard size), 1 = v1 (one link per lane), 2/3 = v2 (one link per
@@ -193,6 +195,15 @@ typedef struct mbd_step_plan {
   const uint64_t* peer_base_ptrs;    /* host array [P]: base address of every rank's symmetric buffer (NULL when P == 1) */
   uint64_t off_rews_words, off_logpd_words, off_partial_words, off_flags_words;  /* flags: 2 rows of 8 words, zeroed */
   uint64_t timeout_cycles;           /* cross-GPU rendezvous timeout in SM cycles; 0 = default (~20 s) */
+  /* ---- batched solves (appended; a zero-initialised plan is one solve, exactly as before) ----
+   * n_solves = S > 1 runs S independent solves (same env, N, H, Ndiffuse, schedule, demo flag; own state_init, key chain,
+   * temperature) in the same three launches.  Every per-solve array then has the solve as its leading axis:
+   * state_init [S, L*13 | 3 | 16], params [S, Nd], ctl [S], Ybars [S, Nd, HNu], rew_hist [S, Nd], Y0s [S, n, HNu],
+   * rews / logpd / weights [S, n], logp [S, N], runs [S, nruns, HNu], partial [S, HNu], scalars [S, 4]; xref is shared.
+   * Batches are single-rank only (P == 1). */
+  int32_t n_solves;                  /* 0 or 1 = one solve */
+  int32_t n_diffuse;                 /* rows per solve of params / Ybars / rew_hist (required, >= 2, when n_solves > 1) */
+  const float* temps_dev;            /* [n_solves] sampling temperatures (required when n_solves > 1; `temp` is then unused) */
 } mbd_step_plan;
 int mbd_step_launch(const mbd_step_plan* plan, mbd_stream s);
 /* the same three launches with CUDA events (mbd_event_create; NULL = skip) recorded before (1), between (1) and (2), between

@@ -42,6 +42,8 @@ class StepPlan(ctypes.Structure):
         ("peer_base_ptrs", ctypes.POINTER(ctypes.c_uint64)),
         ("off_rews_words", ctypes.c_uint64), ("off_logpd_words", ctypes.c_uint64), ("off_partial_words", ctypes.c_uint64),
         ("off_flags_words", ctypes.c_uint64), ("timeout_cycles", ctypes.c_uint64),
+        # batched solves (appended): n_solves 0/1 = one solve; n_diffuse = rows per solve; temps_dev [n_solves]
+        ("n_solves", ctypes.c_int32), ("n_diffuse", ctypes.c_int32), ("temps_dev", c_vp),
     ]
 
 
@@ -100,13 +102,14 @@ def lib():
     L.mbd_event_elapsed_ms.argtypes = [c_vp, c_vp]
     L.mbd_ffma_peak.argtypes = [c_vp, ctypes.c_int, c_f32p, c_vp]
     L.mbd_abi_sizes.argtypes = [c_i32p, ctypes.c_int]
+    L.mbd_abi_batch_offsets.argtypes = [c_i32p, ctypes.c_int]
     _LIB = L
     return L
 
 
 EXPORTS = ["mbd_set_kernel_variant", "mbd_set_prng_layout", "mbd_model_set_warp_order", "mbd_model_set_group_map", "mbd_set_group_stagger", "mbd_layout_info", "mbd_last_error", "mbd_device_count", "mbd_model_create", "mbd_model_destroy", "mbd_sample",
            "mbd_rollout", "mbd_sample_rollout", "mbd_reverse_step", "mbd_car2d_rollout", "mbd_pusht_rollout", "mbd_softmax_weights", "mbd_weighted_sum", "mbd_weighted_sum_runs", "mbd_weighted_sqerr_sum", "mbd_peer_gather", "mbd_test_arith", "mbd_update", "mbd_step_launch", "mbd_step_launch_ev", "mbd_event_create", "mbd_event_destroy", "mbd_event_record",
-           "mbd_event_sync", "mbd_event_elapsed_ms", "mbd_ffma_peak", "mbd_abi_sizes"]
+           "mbd_event_sync", "mbd_event_elapsed_ms", "mbd_ffma_peak", "mbd_abi_sizes", "mbd_abi_batch_offsets"]
 
 
 def check(rc: int, what: str):

@@ -80,6 +80,20 @@ __global__ void k_sample(uint32_t k0, uint32_t k1, uint32_t total, uint32_t begi
   out[i] = sample_elem(k0, k1, idx, total, sigma, Ybar[idx % (uint32_t)HNu]);
 }
 
+// ---- batched solves (mbd_step_plan.n_solves > 1): the solve is blockIdx.y of the fused launch -----------------------
+// Per-solve strides in elements of the arrays that carry a leading solve axis; all zero (and gridDim.y == 1) outside a
+// batched step, so the offsets below vanish.  The noise index stays n_begin + ns inside the solve: solve s draws exactly
+// the noise of a lone solve with its key.
+struct SolveStride { unsigned int state, y0s, n, nd, ybars; };
+template <class St>
+__device__ __forceinline__ void solve_offsets(const SolveStride& z, St*& state, float*& Y0s, float*& rews, float*& logpd,
+                                              const mbd_step_params*& sp, const mbd_step_ctl*& ctl, const float*& Ybars) {
+  const size_t s = blockIdx.y;
+  state += s * z.state; Y0s += s * z.y0s; rews += s * z.n;
+  if (logpd) logpd += s * z.n;
+  sp += s * z.nd; ctl += s; Ybars += s * z.ybars;
+}
+
 // ---- the rollout kernel ----------------------------------------------------------------------------
 struct RolloutArgs {
   const uint32_t* blob;    // device copy of the model blob
@@ -117,15 +131,33 @@ struct RolloutArgs {
   signed char gw[32];
   int count_x;             // group barriers: 32 * (links that are not leaves with contacts), see SyncGroup
   int stagger;             // two-group CTA: cycles group 1 waits before its first step (experiment: de-phase the groups)
+  SolveStride ss;          // batched step: per-solve strides (FUSED kernels only; zero otherwise)
 };
+// the per-solve pointers of a fused rollout launch, formed where they are used: the kernel parameter itself is never
+// written (a written parameter struct is copied to local memory as a whole), and the output pointers are not kept live
+// across the rollout loop (they would cost registers in the single-solve kernels)
+template <bool FUSED>
+__device__ __forceinline__ size_t solve_index() { return FUSED ? (size_t)blockIdx.y : 0; }
+template <bool FUSED>
+struct SolvePtrs {   // blockIdx.y is re-read at every use instead of being held in a register
+  const RolloutArgs& a;
+  __device__ __forceinline__ const float* state_init() const { return a.state_init + solve_index<FUSED>() * a.ss.state; }
+  __device__ __forceinline__ float* Y0s() const { return a.Y0s + solve_index<FUSED>() * a.ss.y0s; }
+  __device__ __forceinline__ float* rews() const { return a.rews + solve_index<FUSED>() * a.ss.n; }
+  __device__ __forceinline__ float* logpd() const { return a.logpd + solve_index<FUSED>() * a.ss.n; }
+};
+template <bool FUSED>
+__device__ __forceinline__ SolvePtrs<FUSED> solve_ptrs(const RolloutArgs& a) { return SolvePtrs<FUSED>{a}; }
 
 __device__ __forceinline__ SampleParams sample_params(const RolloutArgs& a, int HNu) {
   SampleParams q;
   q.k0 = a.k0; q.k1 = a.k1; q.sigma = a.sigma; q.Ybar = a.Ybar;
   if (a.sp != nullptr) {
-    const int i = a.ctl->i;
-    q.k0 = a.sp[i].key[0]; q.k1 = a.sp[i].key[1]; q.sigma = a.sp[i].sigma;
-    q.Ybar = a.Ybars + (size_t)i * HNu;
+    const size_t s = blockIdx.y;   // solve of a batched step (0 otherwise)
+    const mbd_step_params* sp = a.sp + s * a.ss.nd;
+    const int i = a.ctl[s].i;
+    q.k0 = sp[i].key[0]; q.k1 = sp[i].key[1]; q.sigma = sp[i].sigma;
+    q.Ybar = a.Ybars + s * a.ss.ybars + (size_t)i * HNu;
   }
   return q;
 }
@@ -134,6 +166,7 @@ template <bool FUSED, int CMAX>
 __global__ void __launch_bounds__(kRolloutThreads) k_rollout(RolloutArgs a) {
   __shared__ __align__(128) float sblob[MBD_BLOB_WORDS];
   __shared__ __align__(8) uint64_t mbar;
+  const SolvePtrs<FUSED> so = solve_ptrs<FUSED>(a);
   stage_model_tma(sblob, &mbar, a.blob);
   ModelSmem M;
   M.f = sblob;
@@ -155,7 +188,7 @@ __global__ void __launch_bounds__(kRolloutThreads) k_rollout(RolloutArgs a) {
     for (int e = tid; e < cnt; e += kRolloutThreads) {
       int ns = first + e / HNu, j = e % HNu;
       uint32_t idx = (uint32_t)(a.n_begin + ns) * (uint32_t)HNu + (uint32_t)j;
-      a.Y0s[(size_t)ns * HNu + j] = sample_elem(sq.k0, sq.k1, idx, total, sq.sigma, sq.Ybar[j]);
+      so.Y0s()[(size_t)ns * HNu + j] = sample_elem(sq.k0, sq.k1, idx, total, sq.sigma, sq.Ybar[j]);
     }
     __syncthreads();
   }
@@ -172,7 +205,7 @@ __global__ void __launch_bounds__(kRolloutThreads) k_rollout(RolloutArgs a) {
 
   LinkState s;
   {
-    const float* st = a.state_init + (live ? c.l : 0) * MBD_STATE_STRIDE;
+    const float* st = so.state_init() + (live ? c.l : 0) * MBD_STATE_STRIDE;
     s.p = V3(st[0], st[1], st[2]);
     s.q = Q4(st[3], st[4], st[5], st[6]);
     s.w = V3(st[7], st[8], st[9]);
@@ -196,7 +229,7 @@ __global__ void __launch_bounds__(kRolloutThreads) k_rollout(RolloutArgs a) {
     if (live && M.hi(MBD_H_TRACK0 + k) == c.l) my_track = k;
 
   float rsum = 0.0f, tacc = 0.0f;
-  const float* urow = a.Y0s + (size_t)n_rd * HNu;
+  const float* urow = so.Y0s() + (size_t)n_rd * HNu;
   for (int t = 0; t < a.H; ++t) {
     float tau[MBD_MAXDOF];
 #pragma unroll
@@ -246,7 +279,7 @@ __global__ void __launch_bounds__(kRolloutThreads) k_rollout(RolloutArgs a) {
       }
     }
   }
-  if (c.l == 0 && active) a.rews[n_local] = rsum / (float)a.H;
+  if (c.l == 0 && active) so.rews()[n_local] = rsum / (float)a.H;
   if (a.logpd && a.xref) {
     // sum the per-body accumulators in track order on lane 0 of the group
     float tot = 0.0f;
@@ -255,7 +288,7 @@ __global__ void __launch_bounds__(kRolloutThreads) k_rollout(RolloutArgs a) {
       float v = __shfl_sync(0xffffffffu, tacc, src);
       tot += v;
     }
-    if (c.l == 0 && active) a.logpd[n_local] = 0.0f - tot / (float)(ntrack * a.H);
+    if (c.l == 0 && active) so.logpd()[n_local] = 0.0f - tot / (float)(ntrack * a.H);
   }
   if (a.final_state && active && live) {
     float* o = a.final_state + ((size_t)n_local * L + c.l) * MBD_STATE_STRIDE;
@@ -272,6 +305,7 @@ __device__ __forceinline__ void rollout_wpl_body(const RolloutArgs& a, float* sb
   stage_model_tma(sblob, mbar_p, a.blob);
   ModelSmem M;
   M.f = sblob;
+  const SolvePtrs<FUSED> so = solve_ptrs<FUSED>(a);
 
   static_assert(SPLIT == 1 || SPLIT == 2, "links per warp");
   static_assert(SPLIT == 1 || SYNC == 0, "edge barriers assume one link per warp");
@@ -301,7 +335,7 @@ __device__ __forceinline__ void rollout_wpl_body(const RolloutArgs& a, float* sb
     for (int e = tid; e < cnt; e += nthreads) {
       int ns = first + e / HNu, j = e % HNu;
       uint32_t idx = (uint32_t)(a.n_begin + ns) * (uint32_t)HNu + (uint32_t)j;
-      a.Y0s[(size_t)ns * HNu + j] = sample_elem(sq.k0, sq.k1, idx, total, sq.sigma, sq.Ybar[j]);
+      so.Y0s()[(size_t)ns * HNu + j] = sample_elem(sq.k0, sq.k1, idx, total, sq.sigma, sq.Ybar[j]);
     }
     __syncthreads();
   }
@@ -330,7 +364,7 @@ __device__ __forceinline__ void rollout_wpl_body(const RolloutArgs& a, float* sb
 
   LinkState s;
   {
-    const float* st = a.state_init + l * MBD_STATE_STRIDE;
+    const float* st = so.state_init() + l * MBD_STATE_STRIDE;
     s.p = V3(st[0], st[1], st[2]);
     s.q = Q4(st[3], st[4], st[5], st[6]);
     s.w = V3(st[7], st[8], st[9]);
@@ -356,7 +390,7 @@ __device__ __forceinline__ void rollout_wpl_body(const RolloutArgs& a, float* sb
     }
   }
   float rsum = 0.0f, tacc = 0.0f;
-  const float* urow = a.Y0s + (size_t)n_rd * HNu;
+  const float* urow = so.Y0s() + (size_t)n_rd * HNu;
   for (int t = 0; t < a.H; ++t) {
     float tau[MBD_MAXDOF];
 #pragma unroll
@@ -406,7 +440,7 @@ __device__ __forceinline__ void rollout_wpl_body(const RolloutArgs& a, float* sb
       }
     }
   }
-  if (l == 0 && active) a.rews[n_local] = rsum / (float)a.H;
+  if (l == 0 && active) so.rews()[n_local] = rsum / (float)a.H;
   if (a.logpd && a.xref) {
     // per-body accumulators -> shared (reuse E), summed in track order by warp 0
     __syncthreads();  // every warp is done with E
@@ -415,7 +449,7 @@ __device__ __forceinline__ void rollout_wpl_body(const RolloutArgs& a, float* sb
     if (l == 0 && active) {
       float tot = 0.0f;
       for (int k = 0; k < ntrack; ++k) tot += S.E[k * kWplLanes + slot];
-      a.logpd[n_local] = 0.0f - tot / (float)(ntrack * a.H);
+      so.logpd()[n_local] = 0.0f - tot / (float)(ntrack * a.H);
     }
   }
   if (a.final_state && active) {
@@ -484,6 +518,7 @@ __global__ void __launch_bounds__(32 * kPkLinks, 1) k_rollout_pk(RolloutArgs a) 
   __shared__ __align__(128) float sblob[MBD_BLOB_WORDS];
   __shared__ __align__(8) uint64_t mbar;
   extern __shared__ __align__(16) float dyn[];
+  const SolvePtrs<FUSED> so = solve_ptrs<FUSED>(a);
   stage_model_tma(sblob, &mbar, a.blob);
   ModelSmem Ms;
   Ms.f = sblob;
@@ -509,7 +544,7 @@ __global__ void __launch_bounds__(32 * kPkLinks, 1) k_rollout_pk(RolloutArgs a) 
     for (int e = tid; e < cnt; e += nthreads) {
       int ns = first + e / HNu, j = e % HNu;
       uint32_t idx = (uint32_t)(a.n_begin + ns) * (uint32_t)HNu + (uint32_t)j;
-      a.Y0s[(size_t)ns * HNu + j] = sample_elem(sq.k0, sq.k1, idx, total, sq.sigma, sq.Ybar[j]);
+      so.Y0s()[(size_t)ns * HNu + j] = sample_elem(sq.k0, sq.k1, idx, total, sq.sigma, sq.Ybar[j]);
     }
   }
   __syncthreads();   // the duplicated table and (FUSED) this CTA's action rows are complete
@@ -530,7 +565,7 @@ __global__ void __launch_bounds__(32 * kPkLinks, 1) k_rollout_pk(RolloutArgs a) 
 
   pk::State<pk::f2> s;
   {
-    const float* st = a.state_init + l * MBD_STATE_STRIDE;
+    const float* st = so.state_init() + l * MBD_STATE_STRIDE;
     auto b = [&](int i) { return pk::mk2(st[i], st[i]); };
     s.p = pk::mkV(b(0), b(1), b(2));
     s.q = pk::mkQ(b(3), b(4), b(5), b(6));
@@ -547,8 +582,8 @@ __global__ void __launch_bounds__(32 * kPkLinks, 1) k_rollout_pk(RolloutArgs a) 
   __syncthreads();
   if constexpr (SYNC == 2) Y.arrive_pose(l);  // the initial pose is published
   float rsum0 = 0.0f, rsum1 = 0.0f, tacc0 = 0.0f, tacc1 = 0.0f;
-  const float* urow0 = a.Y0s + (size_t)r0 * HNu;
-  const float* urow1 = a.Y0s + (size_t)r1 * HNu;
+  const float* urow0 = so.Y0s() + (size_t)r0 * HNu;
+  const float* urow1 = so.Y0s() + (size_t)r1 * HNu;
   for (int t = 0; t < a.H; ++t) {
     pk::f2 tau[MBD_MAXDOF];
 #pragma unroll
@@ -613,8 +648,8 @@ __global__ void __launch_bounds__(32 * kPkLinks, 1) k_rollout_pk(RolloutArgs a) 
     }
   }
   if (l == 0) {
-    if (act0) a.rews[n0] = rsum0 / (float)a.H;
-    if (act1) a.rews[n0 + 1] = rsum1 / (float)a.H;
+    if (act0) so.rews()[n0] = rsum0 / (float)a.H;
+    if (act1) so.rews()[n0 + 1] = rsum1 / (float)a.H;
   }
   if (a.logpd && a.xref) {
     float* Ef = reinterpret_cast<float*>(S.E);   // per-body accumulators -> shared (reuse E), summed in track order by warp 0
@@ -626,7 +661,7 @@ __global__ void __launch_bounds__(32 * kPkLinks, 1) k_rollout_pk(RolloutArgs a) 
       for (int i = 0; i < 2; ++i) {
         float tot = 0.0f;
         for (int k = 0; k < ntrack; ++k) tot += Ef[k * kPkSamples + 2 * lane + i];
-        if (i == 0 ? act0 : act1) a.logpd[n0 + i] = 0.0f - tot / (float)(ntrack * a.H);
+        if (i == 0 ? act0 : act1) so.logpd()[n0 + i] = 0.0f - tot / (float)(ntrack * a.H);
       }
     }
   }
@@ -660,9 +695,12 @@ struct CarArgs {
   int fused; uint32_t k0, k1; int n_total, n_begin; float sigma; const float* Ybar;
   const mbd_step_params* sp; const mbd_step_ctl* ctl; const float* Ybars;   // device-resident step parameters (see RolloutArgs)
   int prng_part;
+  SolveStride ss;          // batched step: per-solve strides (zero otherwise)
 };
+template <bool BATCH = false>   // BATCH: blockIdx.y is the solve of a batched step
 __global__ void k_car2d(CarArgs a) {
   __shared__ float sp[2 * kCarObs + 4];
+  if constexpr (BATCH) solve_offsets(a.ss, a.x0, a.Y0s, a.rews, a.logpd, a.sp, a.ctl, a.Ybars);
   if (threadIdx.x < 2 * kCarObs + 4) sp[threadIdx.x] = a.params[threadIdx.x];
   __syncthreads();
   int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -1203,6 +1241,14 @@ int mbd_layout_info(int32_t* out, int n) {
   return cnt;
 }
 
+int mbd_abi_batch_offsets(int32_t* out, int n) {
+  const int32_t v[] = {(int32_t)offsetof(mbd_step_plan, n_solves), (int32_t)offsetof(mbd_step_plan, n_diffuse),
+                       (int32_t)offsetof(mbd_step_plan, temps_dev)};
+  const int cnt = (int)(sizeof(v) / sizeof(v[0]));
+  for (int i = 0; i < cnt && i < n; ++i) out[i] = v[i];
+  return cnt;
+}
+
 // sizeof / offsetof of the structs that cross the ABI by pointer (cross-checked against the ctypes mirrors in tests/test_abi.py)
 int mbd_abi_sizes(int32_t* out, int n) {
   const int32_t v[] = {(int32_t)sizeof(mbd_step_params), (int32_t)sizeof(mbd_step_ctl), (int32_t)sizeof(mbd_step_plan),
@@ -1291,7 +1337,8 @@ static int current_device_slot() {
   return dev;
 }
 
-static int launch_rollout(bool fused, mbd::RolloutArgs a, const mbd_model* m, cudaStream_t st) {
+// S > 1: S solves of a batched step in one launch (blockIdx.y = solve, fused only); the selector sees the whole launch
+static int launch_rollout(bool fused, mbd::RolloutArgs a, const mbd_model* m, cudaStream_t st, int S = 1) {
   const int L = m->L;
   {
     int dev = -1;
@@ -1309,14 +1356,16 @@ static int launch_rollout(bool fused, mbd::RolloutArgs a, const mbd_model* m, cu
   //   n <= 148 * 32  one 32-sample CTA per SM, warp per link, named edge barriers, uncapped registers           -> v3
   //   larger         64 samples per SM, two per lane on the packed FFMA2 / FMUL2 / FADD2 path (half the issue slots per
   //                  sample; with the topology in uniform registers it beats the two-group scalar CTA by 8 %)      -> v9
-  if (variant == 0) variant = (L == 11) ? (a.n <= 148 * 8 ? 1 : (a.n <= 148 * 32 ? 3 : ((m->max_ncon <= 2 && m->pk_ok) ? 9 : 2))) : 2;   // contact-heavy models (humanoidstandup): CTA barriers
+  // A batch of S solves is decided on its total sample count S * n (all variants give identical bits).
+  const int ntot = a.n * S;
+  if (variant == 0) variant = (L == 11) ? (ntot <= 148 * 8 ? 1 : (ntot <= 148 * 32 ? 3 : ((m->max_ncon <= 2 && m->pk_ok) ? 9 : 2))) : 2;   // contact-heavy models (humanoidstandup): CTA barriers
   if (!m->named_ok) variant = variant == 3 ? 2 : (variant == 9 ? 8 : variant);   // deep trees: not enough named barriers
   if ((variant == 8 || variant == 9) && !m->pk_ok) variant = 2;   // the packed kernel is built for 11-link hinge-only models (no slide dofs)
   if (variant == 8 || variant == 9) {
     // packed kernel: 64 samples per CTA, two per lane (variant 8: group barriers with decoupled leaves, 9: named edge barriers)
     memcpy(a.wl, m->wl1, sizeof(a.wl));
     a.count_x = 32 * (L - m->nlate);
-    const int grid = (a.n + mbd::kPkSamples - 1) / mbd::kPkSamples;
+    const dim3 grid((a.n + mbd::kPkSamples - 1) / mbd::kPkSamples, S);
     const int dyn = (int)mbd::kPkDynBytes;
 #define MBD_PK_ATTR(F, C, S) CK(cudaFuncSetAttribute(mbd::k_rollout_pk<F, C, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn))
 #define MBD_PK_LAUNCH(C, S)                                                                     \
@@ -1343,13 +1392,15 @@ static int launch_rollout(bool fused, mbd::RolloutArgs a, const mbd_model* m, cu
     memcpy(a.gw, m->gw2, sizeof(a.gw));
     a.count_x = 32 * (L - m->nlate);
     if (split) {
-      int grid = (a.n + 15) / 16, nw = m->nwarps2;
+      const dim3 grid((a.n + 15) / 16, S);
+      const int nw = m->nwarps2;
       if (nw <= 6) MBD_LAUNCH_WPL(6, 4, 0, 2, grid, 32 * nw);     // humanoids: 6 warps, 4 CTAs/SM
       else MBD_LAUNCH_WPL(MBD_MAXL, 1, 0, 2, grid, 32 * nw);
     } else {
-      int grid = (a.n + mbd::kWplLanes - 1) / mbd::kWplLanes;
+      const int gx = (a.n + mbd::kWplLanes - 1) / mbd::kWplLanes;
+      const dim3 grid(gx, S);
       if (L == 11 && variant == 6 && m->max_ncon <= 2) {  // two interleaved 32-sample groups per 704-thread CTA
-        int grid2 = (a.n + 63) / 64;
+        const dim3 grid2((a.n + 63) / 64, S);
         size_t dyn2 = 2 * dyn;
         memcpy(a.wl, m->wl6, sizeof(a.wl));
         a.stagger = g_group_stagger;
@@ -1363,12 +1414,12 @@ static int launch_rollout(bool fused, mbd::RolloutArgs a, const mbd_model* m, cu
         if (fused) mbd::k_rollout_wpl<true, 22, 1, 0, 1, 2, 2><<<grid2, 64 * L, dyn2, st>>>(a);
         else mbd::k_rollout_wpl<false, 22, 1, 0, 1, 2, 2><<<grid2, 64 * L, dyn2, st>>>(a);
       } else if (L == 11 && variant == 2) MBD_LAUNCH_WPL(11, 2, 0, 1, grid, 32 * L);       // CTA-wide barriers
-      else if (L == 11 && variant == 3 && grid <= 148) MBD_LAUNCH_WPL(11, 1, 2, 1, grid, 32 * L);  // one CTA per SM: no register cap
+      else if (L == 11 && variant == 3 && gx * S <= 148) MBD_LAUNCH_WPL(11, 1, 2, 1, grid, 32 * L);  // one CTA per SM (whole launch): no register cap
       else if (L == 11 && variant == 3) MBD_LAUNCH_WPL(11, 2, 2, 1, grid, 32 * L);  // named edge barriers
       else MBD_LAUNCH_WPL(MBD_MAXL, 1, 0, 1, grid, 32 * L);
     }
   } else {
-    int grid = (a.n + mbd::kSPB - 1) / mbd::kSPB;
+    const dim3 grid((a.n + mbd::kSPB - 1) / mbd::kSPB, S);
     if (m->max_ncon <= 2) {
       if (fused) mbd::k_rollout<true, 2><<<grid, mbd::kRolloutThreads, 0, st>>>(a);
       else mbd::k_rollout<false, 2><<<grid, mbd::kRolloutThreads, 0, st>>>(a);
@@ -1460,7 +1511,7 @@ int mbd_car2d_rollout(const float* params_dev, const float* x0_dev, const uint32
   a.fused = key != nullptr;
   a.prng_part = g_prng_part;
   if (key) { a.k0 = key[0]; a.k1 = key[1]; a.n_total = n_total; a.n_begin = n_begin; a.sigma = sigma; a.Ybar = Ybar_dev; }
-  mbd::k_car2d<<<(n_local + 63) / 64, 64, 0, (cudaStream_t)s>>>(a);
+  mbd::k_car2d<false><<<(n_local + 63) / 64, 64, 0, (cudaStream_t)s>>>(a);
   CK(cudaGetLastError());
   return MBD_OK;
 }
@@ -1561,12 +1612,16 @@ static int step_tail_launch(const mbd_step_plan* pl, cudaStream_t st, cudaEvent_
   for (int r = 0; r < pl->P && pl->peer_base_ptrs; ++r) t.peer[r] = reinterpret_cast<float*>(pl->peer_base_ptrs[r]);
   t.off_rews = pl->off_rews_words; t.off_logpd = pl->off_logpd_words; t.off_partial = pl->off_partial_words; t.off_flags = pl->off_flags_words;
   t.timeout_cycles = pl->timeout_cycles ? pl->timeout_cycles : 40000000000ull;   // ~20 s: a dead peer, not a slow one
-  mbd::k_step_weights<<<mbd::kClusterCtas, mbd::kWeightsThreads, 0, st>>>(t);
+  const int S = pl->n_solves > 1 ? pl->n_solves : 1;
+  if (S > 1) { t.temps = pl->temps_dev; t.nd = pl->n_diffuse; }   // one cluster / one z-slice of the update grid per solve
+  if (S > 1) mbd::k_step_weights<true><<<mbd::kClusterCtas * S, mbd::kWeightsThreads, 0, st>>>(t);
+  else mbd::k_step_weights<false><<<mbd::kClusterCtas, mbd::kWeightsThreads, 0, st>>>(t);
   CK(cudaGetLastError());
   if (ev_mid2) CK(cudaEventRecord(ev_mid2, st));
   const int nruns = (pl->n_local + mbd::kTailRun - 1) / mbd::kTailRun;
-  dim3 grid(nruns, (HNu + mbd::kUpdThreads - 1) / mbd::kUpdThreads);
-  mbd::k_step_update<<<grid, mbd::kUpdThreads, 0, st>>>(t);
+  dim3 grid(nruns, (HNu + mbd::kUpdThreads - 1) / mbd::kUpdThreads, S);
+  if (S > 1) mbd::k_step_update<true><<<grid, mbd::kUpdThreads, 0, st>>>(t);
+  else mbd::k_step_update<false><<<grid, mbd::kUpdThreads, 0, st>>>(t);
   CK(cudaGetLastError());
   return MBD_OK;
 }
@@ -1590,6 +1645,20 @@ static int step_launch_impl(const mbd_step_plan* pl, cudaStream_t st, cudaEvent_
   STEP_REQUIRE((uint64_t)pl->n_total * (uint64_t)HNu < 0xffffffffull, "Nsample * H * Nu must stay below 2^32 (threefry counter layout)");
   const bool demo = pl->xref_dev != nullptr;
   STEP_REQUIRE(!demo || (pl->href > 0 && pl->logpd_dev && pl->logpd_all_dev), "demo step needs href, logpd and logpd_all");
+  STEP_REQUIRE(pl->n_solves >= 0, "n_solves must be >= 0");
+  const int S = pl->n_solves > 1 ? pl->n_solves : 1;
+  STEP_REQUIRE(S == 1 || pl->P == 1, "a batch of solves (n_solves > 1) cannot be sharded over ranks (P must be 1)");
+  STEP_REQUIRE(S == 1 || pl->temps_dev != nullptr, "n_solves > 1 needs temps_dev (one temperature per solve)");
+  STEP_REQUIRE(S == 1 || pl->n_diffuse >= 2, "n_solves > 1 needs n_diffuse >= 2 (rows per solve of params / Ybars / rew_hist)");
+  STEP_REQUIRE(S <= 65535, "n_solves exceeds the grid's y / z extent (65535)");
+  // per-solve strides of the arrays with a leading solve axis (all zero for one solve: the kernels then add nothing)
+  mbd::SolveStride ss;
+  memset(&ss, 0, sizeof(ss));
+  if (S > 1) {
+    ss.state = pl->model ? (unsigned)(pl->model->L * MBD_STATE_STRIDE) : (pl->env_kind == MBD_ENV_PUSHT ? (unsigned)MBD_PT_STATE : 3u);
+    ss.y0s = (unsigned)pl->n_local * (unsigned)HNu; ss.n = (unsigned)pl->n_local;
+    ss.nd = (unsigned)pl->n_diffuse; ss.ybars = (unsigned)pl->n_diffuse * (unsigned)HNu;
+  }
 #undef STEP_REQUIRE
   // 1. sampling + rollouts
   if (pl->model) {
@@ -1599,8 +1668,8 @@ static int step_launch_impl(const mbd_step_plan* pl, cudaStream_t st, cudaEvent_
     a.blob = pl->model->blob_dev; a.state_init = pl->state_init_dev; a.Y0s = pl->Y0s_dev; a.n = pl->n_local; a.H = pl->H;
     a.rews = pl->rews_dev; a.xref = pl->xref_dev; a.href = pl->href; a.logpd = demo ? pl->logpd_dev : nullptr;
     a.n_total = pl->n_total; a.n_begin = pl->n_begin;
-    a.sp = pl->params_dev; a.ctl = pl->ctl_dev; a.Ybars = pl->Ybars_dev;
-    int rc = launch_rollout(true, a, pl->model, st);
+    a.sp = pl->params_dev; a.ctl = pl->ctl_dev; a.Ybars = pl->Ybars_dev; a.ss = ss;
+    int rc = launch_rollout(true, a, pl->model, st, S);
     if (rc != MBD_OK) return rc;
   } else if (pl->env_kind == MBD_ENV_PUSHT) {
     if (!pl->car_params_dev || pl->nu != 2 || demo) return MBD_EINVAL;
@@ -1609,8 +1678,8 @@ static int step_launch_impl(const mbd_step_plan* pl, cudaStream_t st, cudaEvent_
     a.params = pl->car_params_dev; a.x0 = pl->state_init_dev; a.Y0s = pl->Y0s_dev; a.n = pl->n_local; a.H = pl->H;
     a.rews = pl->rews_dev;
     a.fused = 1; a.n_total = pl->n_total; a.n_begin = pl->n_begin; a.prng_part = g_prng_part;
-    a.sp = pl->params_dev; a.ctl = pl->ctl_dev; a.Ybars = pl->Ybars_dev;
-    mbd::k_pusht<<<(pl->n_local + 63) / 64, 64, 0, st>>>(a);
+    a.sp = pl->params_dev; a.ctl = pl->ctl_dev; a.Ybars = pl->Ybars_dev; a.ss = ss;
+    mbd::k_pusht<<<dim3((pl->n_local + 63) / 64, S), 64, 0, st>>>(a);
     CK(cudaGetLastError());
   } else {
     if (!pl->car_params_dev || pl->nu != 2) return MBD_EINVAL;
@@ -1619,8 +1688,9 @@ static int step_launch_impl(const mbd_step_plan* pl, cudaStream_t st, cudaEvent_
     a.params = pl->car_params_dev; a.x0 = pl->state_init_dev; a.Y0s = pl->Y0s_dev; a.n = pl->n_local; a.H = pl->H;
     a.rews = pl->rews_dev; a.xref = pl->xref_dev; a.href = pl->href; a.logpd = demo ? pl->logpd_dev : nullptr;
     a.fused = 1; a.n_total = pl->n_total; a.n_begin = pl->n_begin; a.prng_part = g_prng_part;
-    a.sp = pl->params_dev; a.ctl = pl->ctl_dev; a.Ybars = pl->Ybars_dev;
-    mbd::k_car2d<<<(pl->n_local + 63) / 64, 64, 0, st>>>(a);
+    a.sp = pl->params_dev; a.ctl = pl->ctl_dev; a.Ybars = pl->Ybars_dev; a.ss = ss;
+    if (S > 1) mbd::k_car2d<true><<<dim3((pl->n_local + 63) / 64, S), 64, 0, st>>>(a);
+    else mbd::k_car2d<false><<<(pl->n_local + 63) / 64, 64, 0, st>>>(a);
     CK(cudaGetLastError());
   }
   if (ev_mid) CK(cudaEventRecord(ev_mid, st));

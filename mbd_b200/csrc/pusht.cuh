@@ -20,6 +20,7 @@ struct PushTArgs {
   int fused; uint32_t k0, k1; int n_total, n_begin; float sigma; const float* Ybar;
   const mbd_step_params* sp; const mbd_step_ctl* ctl; const float* Ybars;   // device-resident step parameters (see RolloutArgs)
   int prng_part;
+  SolveStride ss;          // batched step: per-solve strides (zero otherwise; mbd_b200.cu)
 };
 
 __device__ __forceinline__ void pt_imp_aref(const float* P, float pos, float vel, float& imp, float& aref) {
@@ -271,6 +272,10 @@ __device__ __forceinline__ float pusht_reward(const float* q) {
 // sample_elem: the planner's per-element sampler (defined in mbd_b200.cu before this header is included)
 __global__ void __launch_bounds__(64) k_pusht(PushTArgs a) {
   __shared__ float P[MBD_PT_NPARAM];
+  {
+    float* no_logpd = nullptr;
+    solve_offsets(a.ss, a.x0, a.Y0s, a.rews, no_logpd, a.sp, a.ctl, a.Ybars);
+  }
   for (int k = threadIdx.x; k < MBD_PT_NPARAM; k += blockDim.x) P[k] = a.params[k];
   __syncthreads();
   const int i = blockIdx.x * blockDim.x + threadIdx.x;

@@ -63,7 +63,25 @@ struct TailArgs {
   int P, rank;
   unsigned long long off_rews, off_logpd, off_partial, off_flags;   // word offsets in the symmetric buffer
   unsigned long long timeout_cycles;
+  // batched solves (one rank): solve s owns row s of every per-solve array (mbd_step_plan layout); nd = Ndiffuse
+  const float* temps;     // [S] or null (one solve: `temp`)
+  int nd;
 };
+
+// Moves every per-solve pointer of `a` to solve s (s = 0: no-op) and takes that solve's temperature.  Each solve then runs
+// exactly the code, and therefore the reduction trees, of a lone solve.
+__device__ __forceinline__ void tail_solve(TailArgs& a, int s) {
+  if (a.temps) a.temp = a.temps[s];
+  const size_t n = (size_t)s * a.n_local, N = (size_t)s * a.N, HNu = a.HNu;
+  const size_t nruns = (a.n_local + kTailRun - 1) / kTailRun;
+  a.sp += (size_t)s * a.nd; a.ctl += s; a.Ybars += (size_t)s * a.nd * HNu;
+  if (a.rew_hist) a.rew_hist += (size_t)s * a.nd;
+  a.Y0s += n * HNu; a.rews += n; a.weights += n;
+  if (a.logpd) a.logpd += n;
+  a.rews_all += N; a.logp += N;
+  if (a.logpd_all) a.logpd_all += N;
+  a.runs += (size_t)s * nruns * HNu; a.partial += (size_t)s * HNu; a.scalars += (size_t)s * 4;
+}
 
 __device__ __forceinline__ void tail_st_release_sys(unsigned int* p, unsigned int v) {
   asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
@@ -136,13 +154,16 @@ __device__ __forceinline__ float cluster_reduce(float v, float* sh, float* slots
 
 // mbd_planner.py:110-127.  One cluster; thread g of the 8192 cluster threads owns the elements i = g (mod 8192): it re-reads
 // only its own elements in every pass, so the passes need no memory barrier beyond the reductions themselves.
+// BATCH: one cluster per solve of a batched step (the single-solve instantiation is the kernel as it was)
+template <bool BATCH>
 __global__ void __cluster_dims__(kClusterCtas, 1, 1) __launch_bounds__(kWeightsThreads, 1) k_step_weights(TailArgs a) {
   __shared__ float sh[32];
   __shared__ float slots[16];
   __shared__ float bcast;
   __shared__ int s_ok;
   cg::cluster_group cl = cg::this_cluster();
-  const int g = (int)cl.block_rank() * kWeightsThreads + threadIdx.x;
+  if constexpr (BATCH) tail_solve(a, (int)(blockIdx.x / kClusterCtas));
+  const int g =(int)cl.block_rank() * kWeightsThreads + threadIdx.x;
   constexpr int G = kClusterCtas * kWeightsThreads;
   const int N = a.N;
   const float fN = (float)N;
@@ -301,9 +322,12 @@ __device__ __forceinline__ float diffusion_update(float Ybar, float Ybar_i, cons
   return Yim1 / p.coef[4];
 }
 
-// grid (nruns, ceil(HNu / 256)); block 256.  ctl->ticket[y]: per column block y; ctl->ticket[MBD_STEP_MAX_COLBLOCKS]: over the column blocks.
+// grid (nruns, ceil(HNu / 256), S); block 256.  ctl->ticket[y]: per column block y; ctl->ticket[MBD_STEP_MAX_COLBLOCKS]: over the
+// column blocks.  Batched: blockIdx.z is the solve, and the tickets and the counter are that solve's.
+template <bool BATCH>
 __global__ void __launch_bounds__(kUpdThreads) k_step_update(TailArgs a) {
   __shared__ int s_flag;
+  if constexpr (BATCH) tail_solve(a, (int)blockIdx.z);
   const int tid = threadIdx.x;
   const int j = blockIdx.y * kUpdThreads + tid;
   const int HNu = a.HNu;

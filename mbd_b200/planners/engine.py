@@ -18,6 +18,7 @@ from __future__ import annotations
 
 import ctypes
 import os
+import types
 from typing import Optional
 
 import numpy as np
@@ -69,17 +70,43 @@ def key_chain(rng_exp, Ndiffuse: int) -> np.ndarray:
     return keys
 
 
+def _is_state_batch(state_init) -> bool:
+    """a list / tuple of states (not a list of numbers, which is one flat state)"""
+    return isinstance(state_init, (list, tuple)) and len(state_init) > 0 and not np.isscalar(state_init[0])
+
+
 class DiffusionEngine:
-    def __init__(self, env, Nsample: int, Hsample: int, temp_sample: float, enable_demo: bool, state_init,
+    def __init__(self, env, Nsample: int, Hsample: int, temp_sample, enable_demo: bool, state_init,
                  device: Optional[torch.device] = None, group=None, Ndiffuse: int = 2, emulate=None):
         """emulate = (P, rank, bufs): rank `rank` of P ranks that all live on THIS device and exchange through the plain
         device buffers `bufs` (one per rank) — the same kernels, flags and peer loads as a real sharded run, used by the
-        single-GPU tests (`make_emulated_ranks`)."""
+        single-GPU tests (`make_emulated_ranks`).
+
+        Batched solves: `state_init` may be a sequence of S states and / or `temp_sample` a sequence of S temperatures (a
+        single value is shared).  The S independent solves then run in the same three launches per step; every per-solve
+        buffer gains a leading solve axis (`solve(s)` gives the views of one solve) and each solve gives exactly the bits it
+        gives alone.  S == 1 is the single-solve engine.  Batches run on one rank only."""
         self.env = env
-        self.N, self.H, self.temp = int(Nsample), int(Hsample), float(temp_sample)
+        states = list(state_init) if _is_state_batch(state_init) else [state_init]
+        temps = [float(t) for t in np.atleast_1d(np.asarray(temp_sample, dtype=np.float64))]
+        S = max(len(states), len(temps))
+        if len(states) == 1:
+            states = states * S
+        if len(temps) == 1:
+            temps = temps * S
+        if len(states) != S or len(temps) != S:
+            raise ValueError(f"{len(states)} initial states but {len(temps)} temperatures")
+        if S > 1 and (emulate is not None or group is not None):
+            raise ops.MbdError("a batch of solves runs on one rank: emulate= / group= are not supported with several solves")
+        self.S, self.temps = S, temps
+        self.N, self.H = int(Nsample), int(Hsample)
+        self.temp = temps[0] if S == 1 else temps
         self.enable_demo = bool(enable_demo)
         self.plan = ShardPlan.from_env(self.N, group) if emulate is None else ShardPlan(self.N, emulate[0], emulate[1], None)
         self.group, self.P, self.rank = group, self.plan.P, self.plan.rank
+        if S > 1 and self.P > 1:
+            raise ops.MbdError("a batch of solves runs on one rank (WORLD_SIZE > 1 shards a single solve instead)")
+        lead = () if S == 1 else (S,)      # leading solve axis of every per-solve buffer
         self.n_local, self.n_begin = self.plan.n_local, self.plan.n_begin
         self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
         self.Nu = env.action_size
@@ -87,7 +114,7 @@ class DiffusionEngine:
         self.Nd = max(int(Ndiffuse), 2)
         d = self.device
         f = dict(device=d, dtype=torch.float32)
-        self.Y0s = torch.empty((self.n_local, self.HNu), **f)
+        self.Y0s = torch.empty(lead + (self.n_local, self.HNu), **f)
         # ---- exchange: P > 1 needs ONE peer-mapped symmetric buffer per rank, [rews n_local | logpd n_local | partial HNu |
         #      2 flag rows of 8 words]; the tail kernels read the peers' slices over NVLink themselves.
         self.sym, self.peer_ptrs = None, None
@@ -116,46 +143,63 @@ class DiffusionEngine:
             self.rews_all = torch.empty(self.N, **f)
             self.logpd_all = torch.empty(self.N, **f) if self.enable_demo else None
         else:
-            self.rews_local = torch.empty(self.n_local, **f)
-            self.logpd_local = torch.empty(self.n_local, **f) if self.enable_demo else None
-            self.partial = torch.empty(self.HNu, **f)
+            self.rews_local = torch.empty(lead + (self.n_local,), **f)
+            self.logpd_local = torch.empty(lead + (self.n_local,), **f) if self.enable_demo else None
+            self.partial = torch.empty(lead + (self.HNu,), **f)
             self.rews_all, self.logpd_all = self.rews_local, self.logpd_local
-        self.weights = torch.empty(self.n_local, **f)
-        self.scalars = torch.zeros(4, **f)
-        self.logp_scratch = torch.empty(self.N, **f)
-        self.run_scratch = torch.empty(((self.n_local + ops.RUN - 1) // ops.RUN) * self.HNu, **f)
+        self.weights = torch.empty(lead + (self.n_local,), **f)
+        self.scalars = torch.zeros(lead + (4,), **f)
+        self.logp_scratch = torch.empty(lead + (self.N,), **f)
+        self.run_scratch = torch.empty(S * ((self.n_local + ops.RUN - 1) // ops.RUN) * self.HNu, **f)
         # ---- device-resident solve state
-        self.Ybars = torch.zeros((self.Nd, self.HNu), **f)        # row i = input of step i, row i-1 = its output (row Nd-1 = YN = 0)
-        self.rew_hist = torch.zeros(self.Nd, **f)                 # rews.mean() of step i
-        self.params = torch.zeros((self.Nd, _lib.STEP_PARAMS_WORDS), device=d, dtype=torch.int32)
-        self.ctl = torch.zeros(_lib.STEP_CTL_WORDS, device=d, dtype=torch.int32)
+        self.Ybars = torch.zeros(lead + (self.Nd, self.HNu), **f)  # row i = input of step i, row i-1 = its output (row Nd-1 = YN = 0)
+        self.rew_hist = torch.zeros(lead + (self.Nd,), **f)        # rews.mean() of step i
+        self.params = torch.zeros(lead + (self.Nd, _lib.STEP_PARAMS_WORDS), device=d, dtype=torch.int32)
+        self.ctl = torch.zeros(lead + (_lib.STEP_CTL_WORDS,), device=d, dtype=torch.int32)
+        self.temps_dev = torch.tensor(temps, **f) if S > 1 else None
         self.launches_per_step = 3
         self.launches_last_step = 3
         self.graph = None
         if env.kind == "xpbd":
             self.model = env.device_model(d)
-            raw = state_init.pipeline_state.raw if hasattr(state_init, "pipeline_state") else state_init
-            self.state_init = torch.as_tensor(np.ascontiguousarray(raw, dtype=np.float32), device=d)
+            self.state_init = self._stack_states(states, lambda st: st.pipeline_state.raw if hasattr(st, "pipeline_state") else st)
             self.xref = torch.as_tensor(env.xref, device=d).contiguous() if self.enable_demo else None
             self.params_car = None
         elif env.kind == "car2d":
             self.model = None
             self.params_car, xref = env.device_params()
-            x0 = state_init.pipeline_state if hasattr(state_init, "pipeline_state") else state_init
-            self.state_init = torch.as_tensor(np.ascontiguousarray(x0, dtype=np.float32), device=d)
+            self.state_init = self._stack_states(states, lambda st: st.pipeline_state if hasattr(st, "pipeline_state") else st)
             self.xref = xref if self.enable_demo else None
         elif env.kind == "pusht":
             if self.enable_demo:
                 raise ValueError("pushT has no demonstration (mbd_planner.py:118 applies to humanoidtrack / car2d)")
             self.model = None
             self.params_car = env.device_params()
-            raw = state_init.pipeline_state.raw if hasattr(state_init, "pipeline_state") else state_init
-            self.state_init = torch.as_tensor(np.ascontiguousarray(raw, dtype=np.float32), device=d)
+            self.state_init = self._stack_states(states, lambda st: st.pipeline_state.raw if hasattr(st, "pipeline_state") else st)
             self.xref = None
         else:
             raise ValueError(env.kind)
         self.rew_xref = float(getattr(env, "rew_xref", 0.0))
         self._plan_c = self._make_plan()
+
+    def _stack_states(self, states, raw_of) -> torch.Tensor:
+        """one state -> its array as today; S states -> [S, ...] (the solve is the leading axis)"""
+        arrs = [np.ascontiguousarray(raw_of(st), dtype=np.float32) for st in states]
+        a = arrs[0] if self.S == 1 else np.ascontiguousarray(np.stack(arrs))
+        return torch.as_tensor(a, device=self.device)
+
+    def solve(self, s: int) -> types.SimpleNamespace:
+        """views of solve s's buffers (with one solve: the buffers themselves)"""
+        if not 0 <= s < self.S:
+            raise IndexError(f"solve {s} of {self.S}")
+        pick = (lambda t: t) if self.S == 1 else (lambda t: None if t is None else t[s])   # noqa: E731
+        return types.SimpleNamespace(Ybars=pick(self.Ybars), rew_hist=pick(self.rew_hist), rews_local=pick(self.rews_local),
+                                     logpd_local=pick(self.logpd_local), weights=pick(self.weights), scalars=pick(self.scalars),
+                                     Y0s=pick(self.Y0s), ctl=pick(self.ctl), state_init=pick(self.state_init), temp=self.temps[s])
+
+    def _single(self, what: str):
+        if self.S > 1:
+            raise ops.MbdError(f"{what} drives one solve; this engine holds a batch of {self.S} (use load_schedule / set_step / step)")
 
     # ---- C-ABI plan ----------------------------------------------------------------------------------------------
     def _make_plan(self) -> "_lib.StepPlan":
@@ -166,7 +210,7 @@ class DiffusionEngine:
         p.state_init_dev = vp(self.state_init)
         p.params_dev, p.ctl_dev, p.Ybars_dev, p.rew_hist_dev = vp(self.params), vp(self.ctl), vp(self.Ybars), vp(self.rew_hist)
         p.n_total, p.n_begin, p.n_local, p.H, p.nu = self.N, self.n_begin, self.n_local, self.H, self.Nu
-        p.temp, p.rew_xref = self.temp, self.rew_xref
+        p.temp, p.rew_xref = self.temps[0], self.rew_xref
         p.xref_dev = vp(self.xref)
         p.env_kind = _lib.ENV_PUSHT if self.env.kind == "pusht" else _lib.ENV_CAR2D
         p.href = 0 if self.xref is None else int(self.xref.shape[1] if self.env.kind == "xpbd" else self.xref.shape[0])
@@ -178,24 +222,31 @@ class DiffusionEngine:
             p.peer_base_ptrs = ctypes.cast(self.peer_ptrs, ctypes.POINTER(ctypes.c_uint64))
         p.off_rews_words, p.off_logpd_words, p.off_partial_words, p.off_flags_words = self.off_rews, self.off_logpd, self.off_partial, self.off_flags
         p.timeout_cycles = int(float(os.environ.get("MBD_XCHG_TIMEOUT_S", "20")) * 2.0e9)
+        p.n_solves, p.n_diffuse, p.temps_dev = self.S, self.Nd, vp(self.temps_dev)
         return p
 
     # ---- solve-level API -----------------------------------------------------------------------------------------
     def load_schedule(self, keys: np.ndarray, sigmas: np.ndarray, alphas: np.ndarray, alphas_bar: np.ndarray):
-        """uploads the per-step parameters of a whole solve: row i = {Y0s_rng of step i, sigmas[i], update_coef(i)}"""
-        Nd = self.Nd
-        if len(sigmas) != Nd or keys.shape != (Nd, 2):
-            raise ops.MbdError(f"schedule of {len(sigmas)} steps does not match the engine (Ndiffuse={Nd})")
+        """uploads the per-step parameters of a whole solve: row i = {Y0s_rng of step i, sigmas[i], update_coef(i)}.
+        A batch takes one key chain per solve, keys [S, Nd, 2] (the schedule is shared)."""
+        Nd, S = self.Nd, self.S
+        keys = np.asarray(keys)
+        if keys.shape == (S, Nd, 2) and S == 1:
+            keys = keys[0]
+        kshape = (Nd, 2) if S == 1 else (S, Nd, 2)
+        if len(sigmas) != Nd or keys.shape != kshape:
+            raise ops.MbdError(f"schedule of {len(sigmas)} steps / keys {keys.shape} do not match the engine (Ndiffuse={Nd}, solves={S})")
         tab = np.zeros((Nd, _lib.STEP_PARAMS_WORDS), np.uint32)
-        tab[:, 0:2] = keys
         tab[:, 2] = np.asarray(sigmas, np.float32).view(np.uint32)
         for i in range(1, Nd):
             tab[i, 3:8] = np.asarray(update_coef(alphas, alphas_bar, i), np.float32).view(np.uint32)
+        tab = np.broadcast_to(tab, keys.shape[:-1] + (_lib.STEP_PARAMS_WORDS,)).copy()
+        tab[..., 0:2] = keys
         self.params.copy_(torch.from_numpy(tab.view(np.int32)))
 
     def set_step(self, i: int):
         """device step counter <- i (the next `step()` runs diffusion step i: reads Ybars[i], writes Ybars[i-1])"""
-        self.ctl[0:1].fill_(int(i))
+        self.ctl.view(-1, _lib.STEP_CTL_WORDS)[:, 0].fill_(int(i))
 
     def step(self):
         """one diffusion step at the device-resident step index (three launches, or one replay of the captured graph)"""
@@ -206,7 +257,7 @@ class DiffusionEngine:
 
     def capture(self):
         """records one step in a CUDA graph; later `step()` calls replay it (parameters come from device memory)"""
-        i0 = int(self.ctl[0].item())
+        i0 = int(self.ctl.view(-1, _lib.STEP_CTL_WORDS)[0, 0].item())
         s = torch.cuda.Stream(device=self.device)
         s.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(s):
@@ -226,7 +277,7 @@ class DiffusionEngine:
     def check_exchange(self):
         """Raises if a cross-GPU rendezvous ever timed out (a peer died or diverged; the outputs are NaN-poisoned).
         Synchronises: call it outside the step loop."""
-        if int(self.ctl[2].item()) != 0:
+        if int(self.ctl.view(-1, _lib.STEP_CTL_WORDS)[:, 2].abs().sum().item()) != 0:
             raise ops.MbdError("cross-GPU rendezvous timed out (a peer rank stopped participating); outputs are NaN")
 
     @classmethod
@@ -258,6 +309,7 @@ class DiffusionEngine:
 
     def rollout_phase(self, key, sigma: float, Ybar_i: torch.Tensor):
         """sampling + rollouts with host-side parameters (path_integral.py's update_once shares it)"""
+        self._single("rollout_phase")
         if self.env.kind == "xpbd":
             ops.sample_rollout(self.model, self.state_init, key, self.N, self.n_begin, self.n_local, self.H, float(sigma), Ybar_i,
                                self.Y0s, self.rews_local, xref=self.xref, logpd_out=self.logpd_local)
@@ -271,6 +323,7 @@ class DiffusionEngine:
 
     def stage_step(self, key, sigma: float, Ybar_i: torch.Tensor, coef, i: int = 1):
         """host-side parameters of ONE step -> row i of the device tables; the next `step()` runs it"""
+        self._single("stage_step")
         row = np.zeros(_lib.STEP_PARAMS_WORDS, np.uint32)
         row[0:2] = np.asarray(key, np.uint32)
         row[2] = np.float32(sigma).view(np.uint32)

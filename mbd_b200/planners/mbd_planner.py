@@ -4,9 +4,15 @@ Same `Args` fields, same recommended-parameter override, same `run_diffusion(arg
 signature, stdout lines and `results/{env}/mu_0ts.npy` artefact; the jitted `reverse_once` is
 replaced by `DiffusionEngine.reverse_once` (hand-written sm_100a CUDA behind the C ABI).
 Under torchrun (WORLD_SIZE > 1) the Nsample axis is sharded over ranks.
+
+`run_diffusion_batch(args_list)` runs several independent solves (own seed and temperature; shared env, sizes, schedule
+and demo flag) as one batch: the S solves share the three launches of every step, and each returns exactly what
+`run_diffusion` returns for it alone.
 """
 from __future__ import annotations
 
+import contextlib
+import io
 import os
 from dataclasses import dataclass
 
@@ -110,39 +116,119 @@ def run_diffusion(args: Args, log_every: int = 10, return_trajectory: bool = Fal
     Yi = Ybars[: args.Ndiffuse - 1].flip(0).reshape(args.Ndiffuse - 1, args.Hsample, Nu)  # jnp.array(Ybars) order
 
     if not args.not_render and _is_main():
-        path = f"{mbd_b200.__path__[0]}/../results/{args.env_name}"
-        if not os.path.exists(path):
-            os.makedirs(path)
-        np.save(f"{path}/mu_0ts.npy", Yi.cpu().numpy())
-        if args.env_name == "car2d":
-            _render_car2d(env, state_init, Yi[-1].cpu().numpy(), args, path)
-        elif env.kind in ("xpbd", "pusht"):
-            # mbd_planner.py:168-178: rollout.html = brax.io.html.render(sys with opt.timestep = env.dt, rollout).  The same
-            # page (and the JSON document inside it, which vis_diffusion.py / brax.io.html.render_from_json consume) is written
-            # by mbd_b200.io.brax_json; rollout_states.npz keeps the plain arrays
-            from ..io import brax_json
-            from ..utils import rollout_states, trajectory_arrays
-            rollout = rollout_states(env.step, state_init, Yi[-1].cpu().numpy())
-            with open(f"{path}/rollout.html", "w") as f:
-                f.write(brax_json.render(env.sys, rollout, env.dt))
-            with open(f"{path}/rollout.json", "w") as f:
-                f.write(brax_json.dumps(env.sys, rollout, env.dt))
-            np.savez(f"{path}/rollout_states.npz", **trajectory_arrays(env, rollout))
+        _save_results(args, env, state_init, Yi)
     rew_final = final_reward(env, engine, Yi[-1])
     if return_trajectory:
         return rew_final, Yi
     return rew_final
 
 
-def final_reward(env, engine: DiffusionEngine, us: torch.Tensor) -> float:
-    """rollout_us(state_init, Yi[-1])[0].mean()  (mbd_planner.py:179-180) — one n=1 launch."""
+# Args fields that every solve of one batch must share (they size the buffers or are part of the shared schedule)
+BATCH_SHARED_FIELDS = ("env_name", "Nsample", "Hsample", "Ndiffuse", "beta0", "betaT", "enable_demo")
+
+
+def _prepare_batch(args_list):
+    """apply_recommended_params to every Args (in place, as run_diffusion does) and check the shared fields; returns the
+    stdout text each call produced, so the caller can print it at the point the sequential loop would.  No GPU call."""
+    args_list = list(args_list)
+    if not args_list:
+        raise ValueError("run_diffusion_batch needs at least one Args")
+    printed = []
+    for a in args_list:
+        buf = io.StringIO()
+        with contextlib.redirect_stdout(buf):
+            apply_recommended_params(a)
+        printed.append(buf.getvalue())
+    for field in BATCH_SHARED_FIELDS:
+        vals = [getattr(a, field) for a in args_list]
+        if any(v != vals[0] for v in vals[1:]):
+            raise ValueError(f"run_diffusion_batch: every solve must share `{field}` (got {vals})")
+    return args_list, printed
+
+
+def run_diffusion_batch(args_list, log_every: int = 10, return_trajectory: bool = False):
+    """`[run_diffusion(a) for a in args_list]` as ONE batch of independent solves on one GPU.
+
+    The solves must agree on env_name, Nsample, Hsample, Ndiffuse, beta0, betaT and enable_demo (after the recommended
+    parameters are applied; ValueError otherwise); each keeps its own seed (reset noise and key chain) and temp_sample.
+    All of them run through one captured graph, three launches per diffusion step.  Returns the list of final rewards, or
+    with return_trajectory the list of (rew_final, Yi) — bit for bit what the sequential loop returns.  Prints the same
+    lines and writes the same results/{env}/ files as that loop (later solves overwrite earlier ones)."""
+    args_list, printed = _prepare_batch(args_list)
+    ops._lib.require_gpu()
+    a0 = args_list[0]
+    env = mbd_b200.envs.get_env(a0.env_name)
+    Nu = env.action_size
+    betas, alphas, alphas_bar, sigmas = make_schedule(a0.beta0, a0.betaT, a0.Ndiffuse)
+    states, keys = [], []
+    for a, text in zip(args_list, printed):
+        # run_diffusion's key handling, solve by solve
+        rng = prng.PRNGKey(seed=a.seed)
+        if _is_main():
+            print(text, end="")
+        rng, rng_reset = prng.split(rng)
+        states.append(env.reset(rng_reset))
+        if _is_main():
+            print(f"init sigma = {sigmas[-1]:.2e}")
+        rng_exp, rng = prng.split(rng)
+        keys.append(key_chain(rng_exp, a.Ndiffuse))
+    S = len(args_list)
+    engine = DiffusionEngine(env, a0.Nsample, a0.Hsample, [a.temp_sample for a in args_list], a0.enable_demo,
+                             states if S > 1 else states[0], Ndiffuse=a0.Ndiffuse)
+    engine.load_schedule(np.stack(keys) if S > 1 else keys[0], sigmas, alphas, alphas_bar)
+    engine.set_step(a0.Ndiffuse - 1)
+    if os.environ.get("MBD_GRAPH", "1") != "0":
+        engine.capture()
+    steps = range(a0.Ndiffuse - 1, 0, -1)
+    pbar = tqdm(steps, desc=f"Diffusing x{S}") if (tqdm is not None and _is_main()) else None
+    for n_done, i in enumerate(pbar if pbar is not None else steps):
+        engine.step()
+        if pbar is not None and (n_done % log_every == log_every - 1 or i == 1):
+            pbar.set_postfix({"rew": f"{engine.solve(0).rew_hist[i].item():.2e}"})
+    out = []
+    for s, a in enumerate(args_list):
+        v = engine.solve(s)
+        Yi = v.Ybars[: a.Ndiffuse - 1].flip(0).reshape(a.Ndiffuse - 1, a.Hsample, Nu)
+        if not a.not_render and _is_main():
+            _save_results(a, env, states[s], Yi)
+        rew_final = final_reward(env, engine, Yi[-1], state_init=v.state_init)
+        out.append((rew_final, Yi) if return_trajectory else rew_final)
+    return out
+
+
+def _save_results(args: Args, env, state_init, Yi: torch.Tensor):
+    """the results/{env}/ artefacts of one solve (mbd_planner.py:157-178)"""
+    path = f"{mbd_b200.__path__[0]}/../results/{args.env_name}"
+    if not os.path.exists(path):
+        os.makedirs(path)
+    np.save(f"{path}/mu_0ts.npy", Yi.cpu().numpy())
+    if args.env_name == "car2d":
+        _render_car2d(env, state_init, Yi[-1].cpu().numpy(), args, path)
+    elif env.kind in ("xpbd", "pusht"):
+        # mbd_planner.py:168-178: rollout.html = brax.io.html.render(sys with opt.timestep = env.dt, rollout).  The same
+        # page (and the JSON document inside it, which vis_diffusion.py / brax.io.html.render_from_json consume) is written
+        # by mbd_b200.io.brax_json; rollout_states.npz keeps the plain arrays
+        from ..io import brax_json
+        from ..utils import rollout_states, trajectory_arrays
+        rollout = rollout_states(env.step, state_init, Yi[-1].cpu().numpy())
+        with open(f"{path}/rollout.html", "w") as f:
+            f.write(brax_json.render(env.sys, rollout, env.dt))
+        with open(f"{path}/rollout.json", "w") as f:
+            f.write(brax_json.dumps(env.sys, rollout, env.dt))
+        np.savez(f"{path}/rollout_states.npz", **trajectory_arrays(env, rollout))
+
+
+def final_reward(env, engine: DiffusionEngine, us: torch.Tensor, state_init: torch.Tensor = None) -> float:
+    """rollout_us(state_init, Yi[-1])[0].mean()  (mbd_planner.py:179-180) — one n=1 launch.  state_init: the device state
+    of one solve of a batched engine (default: the engine's own state)."""
     us = us.reshape(1, engine.H, engine.Nu).contiguous()
+    st = engine.state_init if state_init is None else state_init
     if env.kind == "xpbd":
-        out = ops.rollout(engine.model, engine.state_init, us)
+        out = ops.rollout(engine.model, st, us)
     elif env.kind == "pusht":
-        out = ops.pusht_rollout(engine.params_car, engine.state_init, us)
+        out = ops.pusht_rollout(engine.params_car, st, us)
     else:
-        out = ops.car2d_rollout(engine.params_car, engine.state_init, us)
+        out = ops.car2d_rollout(engine.params_car, st, us)
     return float(out["rews"][0].item())
 
 

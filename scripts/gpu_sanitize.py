@@ -1,6 +1,7 @@
 """Small workloads for compute-sanitizer (racecheck / synccheck / memcheck): every rollout kernel variant on 64 samples x 5
 env steps of humanoidrun (plus hopper for the slide-dof path and the generic instantiation), one full diffusion step (cluster
-statistics kernel + last-CTA update) and two emulated ranks exchanging through peer loads.
+statistics kernel + last-CTA update), two emulated ranks exchanging through peer loads, and a batched step of three solves
+(hopper and humanoidrun: solve axis on every launch, one cluster per solve, per-solve tickets).
     compute-sanitizer --tool racecheck python scripts/gpu_sanitize.py"""
 import os, sys
 import numpy as np, torch
@@ -63,4 +64,15 @@ if which in ("all", "step"):
     torch.cuda.synchronize()
     print("emulated 2-rank steps equal the single-rank ones:", bool(torch.equal(ranks[0].Ybars, e.Ybars) and torch.equal(ranks[1].Ybars, e.Ybars)),
           "err", int(ranks[0].ctl[2].item()), flush=True)
+if which in ("all", "batch"):
+    Nd = 6
+    _, alphas, alphas_bar, sigmas = eng.make_schedule(1e-4, 1e-2, Nd)
+    for name in ("hopper", "humanoidrun"):
+        be = mbd_b200.envs.get_env(name)
+        sts = [be.reset(prng.split(prng.PRNGKey(s))[1]) for s in range(3)]
+        b = eng.DiffusionEngine(be, 100, H, [0.05, 0.1, 0.2], False, sts, Ndiffuse=Nd)
+        b.load_schedule(np.stack([eng.key_chain(np.uint32([s, 9]), Nd) for s in range(3)]), sigmas, alphas, alphas_bar)
+        b.set_step(Nd - 1)
+        b.step(); b.step(); torch.cuda.synchronize()
+        print(f"batched {name} steps done (S=3), ctl.i =", b.ctl[:, 0].tolist(), flush=True)
 print("done")
